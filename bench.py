@@ -38,6 +38,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as build() left it (it may be read-only)
 
 CLOCK_Q = ("index,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.active,"
            "clocks_event_reasons.hw_slowdown,clocks_event_reasons.hw_thermal_slowdown,"
@@ -75,6 +76,7 @@ class ClockSampler(threading.Thread):
                 self.rows.append([c.strip() for c in line.split(",")])
         finally:
             p.terminate()
+            p.wait()    # reaped here, so no exited nvidia-smi outlives the benchmark
 
     def summary(self):
         sm, mx, reasons, pw = [], 0, set(), []
@@ -143,6 +145,43 @@ def make_batch(B, S, seed):
         outs.append(np.ascontiguousarray(v))
         k += 1
     return np.ascontiguousarray(np.concatenate(outs)[:B])
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, sampled):
+    """Writes {name: array} as out_dir/<name>.npy, float32 arrays as float32 and everything else as float64 (exact for
+    the integer outputs).  When they would come to more than DUMP_LIMIT bytes, the arrays named in `sampled` (those
+    whose leading axis is a patch or an image row) keep the same share of that axis, drawn by a fixed seed, so equal
+    shapes give equal positions and two runs stay comparable; the other arrays are written whole."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: v.astype(np.float32 if v.dtype in (np.float16, np.float32) else np.float64) for k, v in arrays.items()}
+    whole = sum(a.nbytes for k, a in arrays.items() if k not in sampled)
+    part = sum(arrays[k].nbytes for k in sampled)
+    share = min(1.0, (DUMP_LIMIT * 15 // 16 - whole) / max(1, part))
+    assert share > 0, "outputs beyond the %d MB dump limit" % (DUMP_LIMIT >> 20)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if name in sampled and share < 1.0:
+            keep = max(1, int(a.shape[0] * share))
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def info_arrays(info):
+    """The tile driver's inst_info_dict as arrays, in instance-id order; contour r = contour[offsets[r]:offsets[r+1]]."""
+    ids = sorted(info)
+    cnt = [np.asarray(info[i]["contour"]).reshape(-1, 2) for i in ids]
+    out = {"inst_id": np.array(ids, np.int64),
+           "inst_bbox": np.array([info[i]["bbox"] for i in ids], np.int64).reshape(-1, 4),
+           "inst_centroid": np.array([info[i]["centroid"] for i in ids], np.float64).reshape(-1, 2),
+           "inst_contour": np.concatenate(cnt) if cnt else np.zeros((0, 2), np.int32),
+           "inst_contour_offsets": np.cumsum([0] + [c.shape[0] for c in cnt])}
+    if ids and info[ids[0]]["type"] is not None:
+        out["inst_type"] = np.array([info[i]["type"] for i in ids], np.int64)
+        out["inst_type_prob"] = np.array([info[i]["type_prob"] for i in ids], np.float64)
+    return out
 
 
 def workload_config(args, world, note=None):
@@ -235,7 +274,7 @@ def run_reference(args):
     cores = os.cpu_count() or 1
     use_cuda_arm = args.ref_forward == "cuda"
     from oracle import postproc_oracle as P
-    P.build()
+    P.lib()                         # libhvo.so as build() left it: no make run inside the tree
     pool = None
     if use_cuda_arm:
         pool = mp.get_context("fork").Pool(cores)  # forked before CUDA is initialised in this process
@@ -312,7 +351,7 @@ def run_reference(args):
 def cpu_baseline(args):
     """All-CPU arm (oracle port of the reference path on every host core), bounded sample -- reported, not the target."""
     from oracle import postproc_oracle as P
-    P.build()
+    P.lib()                         # libhvo.so as build() left it: no make run inside the tree
     arm = CpuArm(args.mode, args.nr_types, args.patch, args.cpu_threads)
     try:
         n = args.cpu_sample or max(2 * arm.procs, 8)
@@ -362,13 +401,16 @@ def run_ours(args):
     d_inst = torch.empty((B, oh, ow), dtype=torch.int32, device=dev)
     d_tab = torch.zeros((B, max_rows, 10), dtype=torch.int64, device=dev)
     d_nr = torch.zeros((B,), dtype=torch.int32, device=dev)
+    # the network's map is written here instead of the library's scratch arena (same kernels, same writes) so that
+    # --dump-outputs can return it as well
+    d_pred = torch.empty((B, oh, ow, oc), dtype=torch.float32, device=dev) if args.dump_outputs else None
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
     pg = PackedGather(ctx, B, max_rows, cap_rows, world, dev)
     torch.cuda.synchronize()
 
     def step_resident():
-        ctx.forward_postproc_dev(d_img.data_ptr(), B, S, S, None, d_inst.data_ptr(), d_tab.data_ptr(), max_rows,
-                                 d_nr.data_ptr())
+        ctx.forward_postproc_dev(d_img.data_ptr(), B, S, S, None if d_pred is None else d_pred.data_ptr(),
+                                 d_inst.data_ptr(), d_tab.data_ptr(), max_rows, d_nr.data_ptr())
         return pg.launch(d_tab, d_nr)     # pack on the library stream + async all_gather (overlaps the next step)
 
     def barrier():
@@ -404,6 +446,11 @@ def run_ours(args):
     got = pg.rows(k)
     assert len(got) == world and all(int(o[-1]) <= cap_rows for o, _ in got), "packed gather payload overflow"
     rows_gathered = int(sum(p.shape[0] for _, p in got))
+    # the last timed step's results on rank 0 as the forward + post-processing call returns them: per patch the
+    # prediction map, the instance map and the instance table padded to max_rows (its first inst_count[b] rows are
+    # the instances), so every shape is fixed by the arguments; the passes below reuse these buffers
+    last = {"pred_map": d_pred.cpu().numpy(), "inst_map": d_inst.cpu().numpy(), "inst_table": d_tab.cpu().numpy(),
+            "inst_count": d_nr.cpu().numpy()} if args.dump_outputs and rank == 0 else None
 
     # ---- e2e through the host-buffer entry point (pinned host buffers), gather included
     h_in = ctx.malloc_host(in_bytes)
@@ -526,6 +573,8 @@ def run_ours(args):
         }
         if not args.no_cpu_baseline and world == 1:
             line["cpu_baseline"] = cpu_baseline(args)
+        if last is not None:
+            dump_outputs(args.dump_outputs, last, sampled=tuple(last))
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -581,6 +630,7 @@ def run_tile(args):
         torch.cuda.synchronize()
         times.append(time.perf_counter() - t0)
     sampler.stop_flag.set()
+    sampler.join(timeout=2)
     t = torch.tensor([float(np.sum(times))], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -602,6 +652,9 @@ def run_tile(args):
                         "note": "host image in, host maps + instance dict out (wall clock, max over ranks)"},
                 "gpu_launches": int(mgr.net.ctx.counter("kernel_launches")), "clocks": sampler.summary(),
                 "instances": len(info), "inst_map_sha1": hashlib.sha1(np.ascontiguousarray(inst).tobytes()).hexdigest()}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dict(pred_map=pred, inst_map=inst, **info_arrays(info)),
+                         sampled=("pred_map", "inst_map"))
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -650,6 +703,7 @@ def run_wsi(args):
     torch.cuda.synchronize()
     t = torch.tensor([time.perf_counter() - t0], dtype=torch.float64, device="cuda")
     sampler.stop_flag.set()
+    sampler.join(timeout=2)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     total = float(t[0])
@@ -697,7 +751,13 @@ def main():
     ap.add_argument("--cpu-threads", type=int, default=32)
     ap.add_argument("--ref-forward", default="cuda", choices=["cpu", "cuda"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32/float64, <= 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "wsi40k"):
+        ap.error("--dump-outputs covers this project's patch and tile4k workloads")
     w = WORKLOADS[args.workload]
     args.stock = args.mode is None and args.nr_types is None and args.batch is None and args.size is None
     args.config = w["config"]
